@@ -411,6 +411,15 @@ def run_reference_arm(args):
     return 0
 
 
+def dump_outputs(path: str, arrays: dict) -> None:
+    """--dump-outputs: each array of wire bytes as path/<name>.npy, one float32 per byte (0..255, exact), so that two builds
+    run with the same arguments (hence the same seeded inputs) can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, raw in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.frombuffer(raw, dtype=np.uint8).astype(np.float32))
+
+
 # ------------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch
@@ -535,6 +544,8 @@ def run_ours(args):
     dev_ms = timed(args.steps, 0)
     launches = sum(e.launch_count() for e in engines) - launches0
     head_got = bytes(finals[(args.steps - 1) % NC][:48].cpu().tolist())
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"msm_result": head_got})
     # the other exchange shapes / transports, timed the same way (all reported; --exchange picks the headline one)
     alts = {}
     if world > 1:
@@ -811,7 +822,14 @@ def _main():
     ap.add_argument("--exchange", default="buckets", choices=["result", "buckets"],
                     help="multi-GPU exchange shape of the headline step (the other one is timed and reported beside it)")
     ap.add_argument("--contexts", type=int, default=4, help="independent steps in flight (streams); 1 = strictly serial")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the MSM result of the last timed step (48-byte compressed G1 point) "
+                         "to DIR/msm_result.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_ours(args)
